@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                   [--config cfg2|cfg3|cfg4|cfg5] [--exchange fused|nccl] [--no-graph] [--no-encoder] [--no-parity]
+                  [--dump-outputs DIR]
 
 Default workload (config.workload) = BASELINE.json configs[1] ("cfg2"): a batch of 256 queries against a 1M x 768
 bf16 corpus, top-32, synthetic data (seeded randn), corpus resident in HBM.  A "step" = one batch through the fused
@@ -318,7 +319,7 @@ def run_search(args, name: str):
         return sh.search(q_dev, k, stream=stream)
 
     for _ in range(max(args.warmup, 3)):
-        step_dev()
+        last_i, last_s = step_dev()
     _barrier(torch, dist, world)
     step_timed = step_dev
     use_graph = args.graph and args.exchange != "nccl"
@@ -326,6 +327,7 @@ def run_search(args, name: str):
         try:
             replay, g_ids, g_sc = sh.capture(q_dev, k)
             step_timed = replay
+            last_i, last_s = g_ids, g_sc
             for _ in range(3):
                 replay()
         except Exception as e:      # pragma: no cover
@@ -350,6 +352,9 @@ def run_search(args, name: str):
         while time.time() < t_end:
             ix.search_dev(q_dev.data_ptr(), nq, k, tmp_s.data_ptr(), tmp_i.data_ptr(), stream=stream)
         torch.cuda.synchronize()
+    # every step writes its answer into the same two buffers and the sampler loop above writes elsewhere: they still
+    # hold what the last timed step returned
+    dump = {"topk_ids": last_i.cpu().numpy().astype(np.float64), "topk_scores": last_s.cpu().numpy()} if args.dump_outputs else None
     ms = _max_over_ranks(torch, dist, world, dev, e0.elapsed_time(e1) / args.steps)
     value = nq / (ms * 1e-3)
 
@@ -477,7 +482,11 @@ def run_search(args, name: str):
         if name == "cfg2" and not args.no_encoder:
             ix.close()
             torch.cuda.empty_cache()
-            out["encoder"] = encoder_leg(local)
+            out["encoder"], emb = encoder_leg(local, args.steps)
+            if dump is not None:
+                dump["encoder_embeddings"] = emb
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.barrier()
@@ -838,11 +847,12 @@ def text_ingest_leg(torch, dist, world, rank, dev, enc, ix, cfg, n_seq, lens, nx
             "text_bytes_per_batch": int(sum(len(t) for t in texts))}
 
 
-def encoder_leg(device: int) -> dict:
+def encoder_leg(device: int, steps: int):
     """Second hot-path row (SURVEY.md 8 a6/a11, BASELINE.json configs[2] shape): bge-base-en
     dimensions, random-init bf16 weights, cfg3 chunk lengths ~N(384, 96) clipped to [16, 512].
-    Device time of the forward (CUDA events inside the library), the same call end to end with
-    host token ids in / host vectors out, and transformers' BertModel on the host cores beside it."""
+    Device time of the forward (CUDA events inside the library) over `steps` batches, the same call end to end with
+    host token ids in / host vectors out, and transformers' BertModel on the host cores beside it.
+    Returns (result, the vectors of the last timed batch)."""
     from aurora_b200.encoder import Encoder, EncoderConfig
 
     cfg = EncoderConfig()
@@ -854,9 +864,9 @@ def encoder_leg(device: int) -> dict:
         for _ in range(3):
             enc.encode_packed(tok, cu)
         dev_ms, e2e_ms = [], []
-        for _ in range(10):
+        for _ in range(steps):
             t0 = time.perf_counter()
-            enc.encode_packed(tok, cu)
+            emb = enc.encode_packed(tok, cu)
             e2e_ms.append((time.perf_counter() - t0) * 1e3)
             dev_ms.append(enc.stats()["total_ms"])
         st = enc.stats()
@@ -896,7 +906,23 @@ def encoder_leg(device: int) -> dict:
                                "sample": f"{n_cpu} chunks, transformers.BertModel fp32 (torch {torch.get_num_threads()} threads), one padded batch ({dt:.2f} s)"}
     except Exception as e:   # transformers missing: report, do not fail the search line
         out["cpu_baseline"] = {"unavailable": str(e)[:120]}
-    return out
+    return out, emb
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: one DIR/<name>.npy per array the timed path returned in its last timed step (ids as float64,
+    exact below 2**53).  The inputs are seeded, so two builds run with the same arguments can be compared output for
+    output."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES} byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def main():
@@ -912,7 +938,11 @@ def main():
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="time plain stream launches instead")
     ap.add_argument("--no-encoder", action="store_true", help="skip the encoder leg of the N=1 cfg2 run")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run oracle check (timing experiments only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy "
+                    "(cfg2 / cfg4: topk_ids, topk_scores, and encoder_embeddings when the encoder leg runs)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config not in ("cfg2", "cfg4")):
+        ap.error("--dump-outputs covers the GPU search arms (cfg2, cfg4)")
     if args.impl == "reference":
         run_reference(args)
     elif args.config in ("cfg2", "cfg4"):

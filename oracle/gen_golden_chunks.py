@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generate tests/golden/chunker_ref.json by running the REAL reference chunker.
+"""Generate tests/golden/chunker_ref.json and chunker_ref_run.json by running the REAL reference chunker.
 
 Test infrastructure.  Run in the authoring container only (``/root/reference`` does not exist on the
 GPU box):  ``python oracle/gen_golden_chunks.py``.  The output is committed; nothing at GPU-test time
@@ -19,6 +19,7 @@ insert_chunks -> WordPiece -> encoder forward -> shard.
 
 from __future__ import annotations
 
+import hashlib
 import importlib.util
 import json
 import os
@@ -26,10 +27,10 @@ import sys
 
 import numpy as np
 
-sys.dont_write_bytecode = True
 REF_FILE = "/root/reference/server/routes/knowledge_base/document_processor.py"
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(os.path.dirname(HERE), "tests", "golden", "chunker_ref.json")
+RUN_OUT = os.path.join(os.path.dirname(HERE), "tests", "golden", "chunker_ref_run.json")
 
 _WORDS = ("alert latency service restart payment database kafka consumer lag rollback deploy canary cpu memory "
           "disk pod node cluster ingress certificate expiry rotate credentials failover replica primary timeout "
@@ -82,6 +83,7 @@ def documents():
 
 
 def main():
+    sys.dont_write_bytecode = True
     mod = load_reference_module()
     out = {"reference_file": "server/routes/knowledge_base/document_processor.py",
            "constants": {"TARGET_CHUNK_SIZE": mod.TARGET_CHUNK_SIZE, "CHUNK_OVERLAP": mod.CHUNK_OVERLAP,
@@ -98,6 +100,28 @@ def main():
     with open(OUT, "w", encoding="utf-8") as f:
         json.dump(out, f, ensure_ascii=False, indent=1)
     print("wrote", OUT)
+    record_run(mod)
+
+
+def input_digest(d) -> str:
+    """SHA-256 of what the chunker is given for one fixture document (text, encoding, file type)."""
+    key = json.dumps([d["text"], d["encoding"], d["file_type"]], ensure_ascii=False).encode("utf-8")
+    return hashlib.sha256(key).hexdigest()
+
+
+def record_run(mod):
+    """Re-run the chunker over the fixture as it was written and store what it returned, keyed by document with the
+    digest of its input: tests/test_chunker_characterisation.py checks the fixture against this record, so the
+    fixture stays pinned to the real chunker's output without the reference tree."""
+    with open(OUT, encoding="utf-8") as f:
+        gold = json.load(f)
+    run = {"reference_file": gold["reference_file"], "documents": []}
+    for d in gold["documents"]:
+        chunks = mod.DocumentProcessor("user-1", f"doc-{d['name']}", d["name"]).process(d["text"].encode(d["encoding"]), d["file_type"])
+        run["documents"].append({"name": d["name"], "input_sha256": input_digest(d), "chunks": chunks})
+    with open(RUN_OUT, "w", encoding="utf-8") as f:
+        json.dump(run, f, ensure_ascii=False, indent=1)
+    print("wrote", RUN_OUT)
 
 
 if __name__ == "__main__":

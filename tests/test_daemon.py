@@ -1,6 +1,9 @@
 """Engine daemon + client shim: the reference's module API over a Unix socket (CPU, test doubles)."""
 
+import shutil
+import tempfile
 import threading
+from pathlib import Path
 
 import pytest
 
@@ -10,9 +13,19 @@ from tests.doubles import HashEmbedder, OracleIndex
 
 
 @pytest.fixture()
-def daemon(tmp_path):
+def sock_dir():
+    """A short directory for the daemon's sockets: a Unix socket path holds at most 107 bytes, and tmp_path under a
+    deep TMPDIR or --basetemp can be longer than that."""
+    base = tempfile.gettempdir()
+    d = tempfile.mkdtemp(prefix="aur-", dir=base if len(base) <= 64 else "/tmp")
+    yield Path(d)
+    shutil.rmtree(d, ignore_errors=True)
+
+
+@pytest.fixture()
+def daemon(sock_dir):
     R.configure(encoder=HashEmbedder(64), capacity=1024, index_factory=lambda dim, cap: OracleIndex(dim, cap))
-    path = str(tmp_path / "kb.sock")
+    path = str(sock_dir / "kb.sock")
     srv = serve(path, background=True)
     yield path
     srv.shutdown(); srv.close_all(final_save=False); srv.server_close()
@@ -47,8 +60,8 @@ def test_client_roundtrip_and_concurrency(daemon):
     assert kb.delete_document_chunks("u", "d") == 3 and kb.search_knowledge_base("u", "redis") == []
 
 
-def test_error_conventions_without_a_daemon(tmp_path):
-    kb = Client(str(tmp_path / "nobody.sock"))
+def test_error_conventions_without_a_daemon(sock_dir):
+    kb = Client(str(sock_dir / "nobody.sock"))
     assert kb.health()["ready"] is False
     assert kb.search_knowledge_base("u", "q") == []
     assert kb.delete_document_chunks("u", "d") == -1 and kb.delete_user_chunks("u") == -1
@@ -78,7 +91,7 @@ def test_bootstrap_requires_its_variables(monkeypatch):
     assert bootstrap._model_config("minilm-l6").hidden == 384
 
 
-def test_socket_is_private_and_facade_and_learn_over_the_wire(tmp_path):
+def test_socket_is_private_and_facade_and_learn_over_the_wire(sock_dir):
     import os
     import stat
 
@@ -87,7 +100,7 @@ def test_socket_is_private_and_facade_and_learn_over_the_wire(tmp_path):
 
     R.configure(encoder=HashEmbedder(64), capacity=1024, index_factory=lambda dim, cap: OracleIndex(dim, cap))
     K.configure(encoder=HashEmbedder(64), capacity=256, index_factory=lambda dim, cap: OracleIndex(dim, cap), org_resolver=lambda u: "acme")
-    path = str(tmp_path / "kb.sock")
+    path = str(sock_dir / "kb.sock")
     srv = serve(path, background=True, learn_module=K)
     try:
         assert stat.S_IMODE(os.stat(path).st_mode) == 0o600            # any process that can open it reads every tenant
@@ -109,19 +122,19 @@ def test_socket_is_private_and_facade_and_learn_over_the_wire(tmp_path):
         srv.shutdown(); srv.close_all(final_save=False); srv.server_close()
         R.configure(factory=lambda: (_ for _ in ()).throw(RuntimeError("backend down")))
         K.configure(factory=lambda: (_ for _ in ()).throw(RuntimeError("backend down")), org_resolver=lambda u: None)
-    off = Client(str(tmp_path / "gone.sock"))
+    off = Client(str(sock_dir / "gone.sock"))
     assert off.store_good_rca("a", "i", "f", "t", "s", "g", "c", "s", [], []) is False and off.search_similar_good_rcas("a", "t", "s", "g") == []
     assert off.delete_incident_knowledge("a", "i") is False and off.delete_user_knowledge("a") == -1
     with pytest.raises(Exception):
         off._get_weaviate_client()
 
 
-def test_concurrent_searches_are_coalesced_into_encoder_batches(tmp_path):
+def test_concurrent_searches_are_coalesced_into_encoder_batches(sock_dir):
     """64 client threads, one query each at a time (the reference's call pattern): the daemon gathers them into a few
     encoder batches instead of 64 x N single-sequence forwards, and every caller still gets exactly its own answer."""
     emb = HashEmbedder(64)
     R.configure(encoder=emb, capacity=4096, index_factory=lambda dim, cap: OracleIndex(dim, cap))
-    path = str(tmp_path / "kb.sock")
+    path = str(sock_dir / "kb.sock")
     srv = serve(path, background=True, coalesce_us=20000)
     try:
         kb = Client(path)
@@ -152,13 +165,13 @@ def test_concurrent_searches_are_coalesced_into_encoder_batches(tmp_path):
         R.configure(factory=lambda: (_ for _ in ()).throw(RuntimeError("backend down")))
 
 
-def test_snapshot_policy_saves_and_restores(tmp_path):
+def test_snapshot_policy_saves_and_restores(tmp_path, sock_dir):
     import os
 
     emb = HashEmbedder(64)
     R.configure(encoder=emb, capacity=1024, index_factory=lambda dim, cap: OracleIndex(dim, cap))
     snap = str(tmp_path / "snap")
-    path = str(tmp_path / "kb.sock")
+    path = str(sock_dir / "kb.sock")
     srv = serve(path, background=True, snapshot_dir=snap, save_every=3, save_seconds=3600)
     try:
         kb = Client(path)
@@ -186,7 +199,7 @@ def json_meta(snap):
     return json.load(open(os.path.join(snap, "meta.json")))
 
 
-def test_daemon_crash_between_snapshots_loses_nothing_acknowledged(tmp_path):
+def test_daemon_crash_between_snapshots_loses_nothing_acknowledged(tmp_path, sock_dir):
     """The deployment's durability story end to end (CPU doubles): a daemon with a snapshot directory and the mutation
     log takes a snapshot, acknowledges more inserts and a delete, and dies without saving; the next daemon restores
     the snapshot, replays the log and serves exactly what the first one had acknowledged."""
@@ -205,7 +218,7 @@ def test_daemon_crash_between_snapshots_loses_nothing_acknowledged(tmp_path):
         return kb
 
     R.configure(factory=make)
-    path = str(tmp_path / "kb.sock")
+    path = str(sock_dir / "kb.sock")
     srv = serve(path, background=True, snapshot_dir=snap, save_every=10 ** 9, save_seconds=10 ** 9)
     try:
         kb = Client(path)
@@ -220,7 +233,7 @@ def test_daemon_crash_between_snapshots_loses_nothing_acknowledged(tmp_path):
     finally:
         srv.shutdown(); srv.close_all(final_save=False); srv.server_close()          # "crash": no final snapshot
     R.configure(factory=make)                                                          # a new process would start like this
-    path2 = str(tmp_path / "kb2.sock")
+    path2 = str(sock_dir / "kb2.sock")
     srv2 = serve(path2, background=True, snapshot_dir=snap, save_every=10 ** 9, save_seconds=10 ** 9)
     try:
         kb2 = Client(path2)
